@@ -301,7 +301,14 @@ def main():
     ap.add_argument("--text-in", action="store_true", help="(kept for compatibility: the text-in leg is on by default at N=1)")
     ap.add_argument("--text-docs", type=int, default=8192)
     ap.add_argument("--text-bytes", type=int, default=2048)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the picks of the last timed step as DIR/picks.npy (float64, one per request of the batch; rank 0), "
+                         "so that two builds can be compared on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "smgx":
+        ap.error("--dump-outputs applies to --impl smgx")
     args.warmup = max(args.warmup, 3)
 
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
@@ -422,8 +429,14 @@ def main():
         h.call("smgx_timer_stop_ms", 0, C.byref(ms)) if one_lane else h.call("smgx_timer_stop_all_ms", C.byref(ms))
         (region_ms if gated else region_ms_ungated).append(float(ms.value))
         gpu_launches = pol.kernel_launches() - launches0   # the hold kernel is not counted: it is not part of the path
+        last_slot = order[-1]
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        picks = np.zeros(B, np.int32)
+        h.call("smgx_memcpy_d2h", picks.ctypes.data_as(C.c_void_p), d_out[last_slot], B * 4)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "picks.npy"), picks.astype(np.float64))
     ms_med = float(np.median(region_ms))
     t_dev = max_over_ranks(ms_med / 1e3)
     value = world * args.steps * B / t_dev

@@ -9,6 +9,7 @@ import pytest
 
 from oracle import bpe_ref, orc
 from smg_b200 import synth
+from tests import random_vectors as RV
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -35,17 +36,27 @@ def test_golden_vectors_on_gpu():
     assert tok.encode("") == [] and tok.encode("<|endoftext|>") == [g["specials"]["<|endoftext|>"]]
 
 
-def test_random_text_vs_oracle_and_live_tiktoken():
-    pol, tok, g = _policy_and_tok()
-    ranks = bpe_ref.load_tiktoken_bpe(VOCAB)
-    enc = bpe_ref.CoreBPE(ranks, g["specials"])
+def random_tiktoken_texts():
     rng = random.Random(5)
     alphabet = "abcdefghij XYZ 0123\n\t\r'.,!?-_()<|>im_startend" + "éß你好\U0001f44b 　ſ"
     texts = ["".join(rng.choice(alphabet) for _ in range(rng.randint(0, 300))) for _ in range(600)]
     texts += ["word " * 500, "x" * 3000, " " * 2000 + "end", "\n".join("line %d: the quick brown fox" % i for i in range(200))]
+    return texts
+
+
+def test_random_text_vs_oracle_and_live_tiktoken():
+    """Against the oracle, the ids tiktoken gave for these texts (tests/golden/random_vectors.json, written by
+    tests/golden/gen_random_vectors.py), and live tiktoken when it is importable."""
+    pol, tok, g = _policy_and_tok()
+    ranks = bpe_ref.load_tiktoken_bpe(VOCAB)
+    enc = bpe_ref.CoreBPE(ranks, g["specials"])
+    texts = random_tiktoken_texts()
     got = tok.encode_batch(texts)
-    for t, ids in zip(texts, got):
+    want = RV.load("tiktoken_gpu_texts")
+    assert len(want) == len(texts)
+    for t, ids, w in zip(texts, got, want):
         assert ids == enc.encode_with_special_tokens(t), repr(t[:80])
+        assert RV.ids_digest(ids) == w, repr(t[:80])
     try:
         import tiktoken
     except ImportError:
@@ -137,18 +148,32 @@ def test_hf_tokenizer_json_matches_tokenizers_crate(fixture):
         assert ids == want, repr(t[:80])
 
 
-def test_hf_tokenizer_live_tokenizers_random_texts():
-    tokenizers = pytest.importorskip("tokenizers")
-    from smg_b200 import CacheAwareConfig, CacheAwarePolicy
-    path = os.path.join(GOLD, "hf_llama3_style_tokenizer.json")
-    ref = tokenizers.Tokenizer.from_file(path)
-    pol = CacheAwarePolicy(CacheAwareConfig(eviction_interval_secs=0))
-    tok = pol.load_hf_tokenizer(path)
+def random_hf_texts():
     rng = random.Random(9)
     alphabet = "abcdefghij the quick XYZ 0123456789\n\t\r'.,!?-_(){}[]<|>eot_idbegin_of_text" + "éßüï你好世界\U0001f44b\U0001f30d ١٢٣"
     texts = ["".join(rng.choice(alphabet) for _ in range(rng.randint(0, 400))) for _ in range(400)]
     texts += ["<|begin_of_text|>" + "hello world " * 50 + "<|eot_id|>", "don't DON'T I'LL we'Ve 'S", "   \n\n  \n x  \n", "12345678901234567890"]
+    return texts
+
+
+def test_hf_tokenizer_live_tokenizers_random_texts():
+    """Against the ids the `tokenizers` package gave for these texts (tests/golden/random_vectors.json, written by
+    tests/golden/gen_random_vectors.py), and against the live package when it is importable."""
+    from smg_b200 import CacheAwareConfig, CacheAwarePolicy
+    path = os.path.join(GOLD, "hf_llama3_style_tokenizer.json")
+    pol = CacheAwarePolicy(CacheAwareConfig(eviction_interval_secs=0))
+    tok = pol.load_hf_tokenizer(path)
+    texts = random_hf_texts()
     got = tok.encode_batch(texts)
+    want = RV.load("hf_llama3_style_texts")
+    assert len(want) == len(texts)
+    for t, a, b in zip(texts, got, want):
+        assert RV.ids_digest(a) == b, repr(t[:80])
+    try:
+        import tokenizers
+    except ImportError:
+        return
+    ref = tokenizers.Tokenizer.from_file(path)
     want = [e.ids for e in ref.encode_batch(texts, add_special_tokens=False)]
     for t, a, b in zip(texts, got, want):
         assert a == b, repr(t[:80])

@@ -7,6 +7,7 @@ import struct
 import pytest
 
 from oracle import orc
+from tests import random_vectors as RV
 from tests import scenarios_event_tree as S
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -51,14 +52,28 @@ def test_xxh3_golden_vectors():
         assert orc.xxh3_64(data, c["seed"]) == int(c["digest"]), (len(data), c["seed"])
 
 
-def test_xxh3_against_live_xxhash_if_present():
-    xxhash = pytest.importorskip("xxhash")
+def xxh3_random_inputs():
+    """Seeded random byte strings of every length 0..299 and a few long ones, then 16 token ids."""
     import random
     rng = random.Random(7)
-    for n in list(range(0, 300)) + [1023, 1024, 1025, 4096, 10000]:
-        d = bytes(rng.getrandbits(8) for _ in range(n))
-        assert orc.xxh3_64(d, 1337) == xxhash.xxh3_64_intdigest(d, seed=1337)
+    data = [bytes(rng.getrandbits(8) for _ in range(n)) for n in list(range(0, 300)) + [1023, 1024, 1025, 4096, 10000]]
     toks = [rng.getrandbits(32) for _ in range(16)]
+    return data, toks
+
+
+def test_xxh3_against_live_xxhash_if_present():
+    """Against the digests Python `xxhash` gave for these inputs (tests/golden/random_vectors.json, written by
+    tests/golden/gen_random_vectors.py), and against the live package when it is importable."""
+    data, toks = xxh3_random_inputs()
+    want = RV.load("xxh3_seed1337")
+    assert [orc.xxh3_64(d, 1337) for d in data] == [int(x) for x in want["digests"]]
+    assert orc.compute_content_hash(toks) == int(want["content_hash"])
+    try:
+        import xxhash
+    except ImportError:
+        return
+    for d in data:
+        assert orc.xxh3_64(d, 1337) == xxhash.xxh3_64_intdigest(d, seed=1337)
     assert orc.compute_content_hash(toks) == xxhash.xxh3_64_intdigest(struct.pack("<16I", *toks), seed=1337)
 
 
